@@ -2,6 +2,7 @@
 """bench.py -- candidate 3-LUT tuples/s of the `--lut` search path (BASELINE.json's metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--gates n]
+                  [--dump-outputs DIR]
 
 A STEP is one pass of the hot path -- search_5lut followed by search_7lut (lut.c:553,593) -- over a
 batch of synthetic search states shaped like the ones `sboxgates --lut -o 0 rijndael.txt` presents
@@ -26,6 +27,14 @@ and merged on the devices, one all-reduce(MIN) per search phase), with the one-G
 search beside it and the results compared in the run -- strong scaling of north_star's partition.
 Further records on one GPU: `replay` (recorded real calls of seeded reference runs through the C
 ABI, results asserted), `graph` (wall-clock to graph: the drop-in CLI on BASELINE.json configs[1]).
+
+--dump-outputs DIR writes the result structs the last timed step returned (sbg_search_batch, one row
+per search state) as float64 arrays: DIR/r5.npy and DIR/r7.npy (search_5lut / search_7lut, columns
+RESULT_COLUMNS) and DIR/node.npy (NODE_COLUMNS); 64-bit keys are split into two exact 32-bit halves.
+The states of a step depend only on --gates, --batch and the step's number (seed 1000 + s, warm-up
+steps counted), so
+the same arguments give the same inputs in every run and two builds can be compared file by file.
+With N > 1 every rank writes its own states' results, with the suffix _rank<r>.
 
 --impl reference times the reference's own object code (oracle/_ref/libsbgref.so, built from the
 unmodified sources; the oracle port if that is absent) on the host cores, one process per core, each
@@ -136,6 +145,30 @@ def build_batch(n, batch, step_seed):
                         mask=_mux_mask(fixed), inbits=[b for b, _ in fixed], order5=o5, outer=oo,
                         middle=om))
     return out
+
+
+RESULT_COLUMNS = ("found", "ordering", "pos_outer", "pos_middle", "func_outer", "func_middle",
+                  "func_inner", "inner_seen", "gate0", "gate1", "gate2", "gate3", "gate4", "gate5",
+                  "gate6", "stale_outer", "index", "key_hi", "key_lo", "tuples_feasible",
+                  "tuples_swept")
+NODE_COLUMNS = ("found_stage", "gate0", "gate1", "gate2", "func3", "seen3", "key3_hi", "key3_lo")
+
+
+def _result_row(r):
+    return [r.found, r.ordering, r.pos_outer, r.pos_middle, r.func_outer, r.func_middle,
+            r.func_inner, r.inner_seen] + list(r.gates) + [
+        r.stale_outer, r.index, r.key >> 32, r.key & 0xFFFFFFFF, r.tuples_feasible, r.tuples_swept]
+
+
+def dump_outputs(out_dir, results, suffix=""):
+    """The SbgNodeResult structs of one sbg_search_batch call as float64 arrays (every field is an
+    integer below 2**53 once the keys are split, so the values are exact)."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"r5": [_result_row(r.r5) for r in results], "r7": [_result_row(r.r7) for r in results],
+              "node": [[r.found_stage] + list(r.gates3) + [r.func3, r.seen3, r.key3 >> 32,
+                                                           r.key3 & 0xFFFFFFFF] for r in results]}
+    for name, rows in arrays.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), np.array(rows, dtype=np.float64))
 
 
 def units_of(n, r5, r7):
@@ -441,7 +474,11 @@ def main():
     ap.add_argument("--sharded-gates", default="64h,96,128",
                     help="state sizes of the tuple-space sharding record; suffix h = one mux level "
                          "deep (128 masked positions) instead of the full mask")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the results of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -601,10 +638,12 @@ def main():
         acc["h2d"], acc["d2h"] = tr1[0] - tr0[0], tr1[1] - tr0[1]
         acc["gather_ms"] = gather_ms
         acc["ranks_compute"] = ranks_compute
-        return max(ranks_ms), ranks_ms, acc, clocks
+        return max(ranks_ms), ranks_ms, acc, clocks, results[-1]
 
-    ms_res, ranks_res, acc_res, clocks = timed(resident=True)
-    ms_e2e, ranks_e2e, acc_e2e, _ = timed(resident=False)
+    ms_res, ranks_res, acc_res, clocks, last_results = timed(resident=True)
+    ms_e2e, ranks_e2e, acc_e2e, _, _ = timed(resident=False)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_results, "_rank%d" % rank if world > 1 else "")
 
     # kernel families in isolation (one state at a time, CUDA events between the kernels): the
     # dominant kernel's launch durations for the roofline; not part of `value`

@@ -20,12 +20,18 @@ Produces
   tests/golden/order_tables.json          the literal 70-row table of lut.c:396-415
   tests/golden/xml_names.json             output file names (gate count + Speck fingerprint,
                                           state.c:123-125) of seeded end-to-end reference runs
+  tests/golden/ref_checks.json            the reference's struct layout, its answers to the seeded
+                                          random searches of _support.random_ref_cases, and the
+                                          graphs (XML as written, DOT from its -d converter) of
+                                          seeded CLI runs
+  tests/golden/sboxes/*.txt               the reference's S-box tables (data inputs of its CLI)
 """
 import argparse
 import glob
 import json
 import os
 import re
+import shutil
 import struct
 import subprocess
 import sys
@@ -308,17 +314,66 @@ def literal_order_table():
     return [nums[7 * i:7 * i + 7] for i in range(70)]
 
 
+# seeded reference CLI runs whose graphs ref_checks.json stores: (S-box, options, seed, keep only
+# the last file written)
+CLI_GRAPHS = [("crypto1_fa.txt", ["-l"], "seed1", False), ("crypto1_fc.txt", ["-l"], "seed1", False),
+              ("crypto1_fc.txt", ["-l"], "seed2", False), ("des_s1.txt", ["-o", "0"], "seed1", True)]
+
+
+def ref_checks():
+    """What tests/test_oracle_ref.py compares with, taken from the reference's own object code."""
+    import ctypes as C
+    lib = S.ref_lib()
+    a, b, c, d, e = (C.c_int() for _ in range(5))
+    lib.sbgref_sizes(C.byref(a), C.byref(b), C.byref(c), C.byref(d))
+    layout = {"ttable": a.value, "gate": b.value, "state": c.value, "state_gates_offset": d.value}
+    lib.sbgref_options_layout(C.byref(a), C.byref(b), C.byref(c), C.byref(d), C.byref(e))
+    layout.update({"options_randomize_offset": a.value, "options_lut_graph_offset": b.value,
+                   "options_verbosity_offset": c.value, "options": d.value, "boolfunc": e.value})
+    searches = []
+    for which, tabs, tgt, mask, inb, seed in S.random_ref_cases():
+        rng = S.OrcRng.from_seed(seed)
+        found, ret, draws = S.ref_search(which, tabs, tgt, mask, inb, rng)
+        searches.append({"which": which, "found": int(found), "ret": ret, "draws": draws,
+                         "rng_after": [str(w) for w in rng.words()], "rng_p": rng.p})
+    graphs = []
+    exe = os.path.join(REFDIR, "sboxgates_ref")
+    for sbox, cli, seed, last_only in CLI_GRAPHS:
+        with tempfile.TemporaryDirectory() as tmp:
+            env = dict(os.environ, SBG_SEEDFILE=os.path.join(GOLD, seed + ".bin"))
+            subprocess.run([exe] + cli + [os.path.join(REFDIR, "sboxes", sbox)], cwd=tmp, env=env,
+                           check=True, stdout=subprocess.DEVNULL, timeout=300)
+            names = sorted(os.path.basename(p) for p in glob.glob(os.path.join(tmp, "*.xml")))
+            files = []
+            for name in names[-1:] if last_only else names:
+                xml = open(os.path.join(tmp, name)).read()
+                dot = subprocess.run([exe, "-d", name], cwd=tmp, env=env, check=True,
+                                     capture_output=True, text=True).stdout
+                files.append({"name": name, "xml": xml, "dot": dot})
+        graphs.append({"key": " ".join([sbox] + cli + [seed]), "names": names, "files": files})
+    json.dump({"layout": layout, "searches": searches, "graphs": graphs},
+              open(os.path.join(GOLD, "ref_checks.json"), "w"), indent=1)
+    os.makedirs(os.path.join(GOLD, "sboxes"), exist_ok=True)
+    for path in sorted(glob.glob(os.path.join(REF, "sboxes", "*.txt"))):
+        shutil.copyfile(path, os.path.join(GOLD, "sboxes", os.path.basename(path)))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--skip-runs", action="store_true", help="keep existing run_*.bin files")
     ap.add_argument("--only-stale", action="store_true", help="just print the stale-cache cases")
+    ap.add_argument("--only-ref-checks", action="store_true",
+                    help="only tests/golden/ref_checks.json and tests/golden/sboxes/")
     args = ap.parse_args()
     os.makedirs(GOLD, exist_ok=True)
     if not S.ref_available():
-        sys.exit("oracle/_ref is not built: run `make -C oracle` where /root/reference exists")
+        sys.exit("oracle/_ref is not built: run `make -C oracle` where the reference sources are")
 
     if args.only_stale:
         print(len(find_stale_cache_cases()))
+        return
+    if args.only_ref_checks:
+        ref_checks()
         return
     for i in (1, 2):
         with open(os.path.join(GOLD, "seed%d.bin" % i), "wb") as fp:
@@ -362,6 +417,7 @@ def main():
 
     json.dump(primitives(np.random.RandomState(3)), open(os.path.join(GOLD, "primitives.json"), "w"))
     json.dump(literal_order_table(), open(os.path.join(GOLD, "order_tables.json"), "w"))
+    ref_checks()
     print("done")
 
 

@@ -330,7 +330,7 @@ def synthetic_state(n, seed, num_inputs=8):
 
 def rijndael_sbox():
     """The AES S-box from its definition (inverse in GF(2^8) mod x^8+x^4+x^3+x+1, then the affine
-    map); equals sboxes/rijndael.txt, which tests/test_oracle_ref.py checks when it is present."""
+    map); equals sboxes/rijndael.txt (tests/golden/sboxes/), which tests/test_oracle_ref.py checks."""
     def mul(a, b):
         r = 0
         while b:
@@ -374,6 +374,24 @@ def oracle_check(num, target, mask, tables):
     mask, mp = _u64(mask)
     tabs, tp = _u64(np.stack(tables))
     return bool(lib.orc_check_n_lut_possible(num, gp, mp, tp))
+
+
+def random_ref_cases():
+    """The 30 x 2 seeded random searches tests/golden/ref_checks.json holds the reference's answers
+    to: yields (which, tables, target, mask, inbits, seed bytes) in the order they were recorded."""
+    sbox = rijndael_sbox()
+    rs = np.random.RandomState(123)
+    for i in range(30):
+        n = int(rs.choice([7, 8, 9, 10, 11]))
+        tabs = synthetic_state(n, seed=3000 + i, num_inputs=min(8, n))
+        pos = rs.choice(256, int(rs.choice([6, 10, 16, 24, 40])), replace=False)
+        mask = np.zeros(4, dtype=np.uint64)
+        for p in pos:
+            mask[p >> 6] |= np.uint64(1) << np.uint64(p & 63)
+        tgt = sbox_target(sbox, int(rs.randint(0, 8)))
+        inb = [int(rs.randint(0, min(8, n)))] if i % 3 == 0 else []
+        for which in (5, 7):
+            yield which, tabs, tgt, mask, inb, rs.bytes(128)
 
 
 def oracle_get_lut_function(in1, in2, in3, target, mask, rng, randomize=True):
